@@ -294,6 +294,8 @@ def build_recipe_model(wl, enc, llm, lora, world):
                          lora_dropout=0.0, inference_mode=False)))
     model_config = OmegaConf.create(dict(llm_name=wl["llm"], llm_path=tmp, llm_dim=llm.d, encoder_name="whisper", encoder_path=wl["enc"], encoder_dim=enc.d,
                                          encoder_projector="linear", encoder_projector_ds_rate=5, b200_random_init=True))
+    torch.cuda.manual_seed(train_config.seed)                      # as finetune.main does: the projector's nn.Linear init draws from the global RNG
+    torch.manual_seed(train_config.seed)
     encoder = setup_encoder(train_config, model_config)
     llm_mod = setup_llm(train_config, model_config)
     projector = setup_encoder_projector(train_config, model_config)
@@ -560,6 +562,23 @@ def measure_gemm_traffic(workload, budget_s=240.0):
     return round(sum(per.values()) / len(per)), f"measured in this run: ncu child process, one eager step of the same workload, {len(per)} GEMM launches"
 
 
+def dump_outputs(out_dir, loss, acc, eng, sample=1 << 22):
+    """What the last timed step hands its caller, as float32 .npy files: the loss and the token accuracy it returns, and the trainable
+    parameters after its AdamW update (every trainable, concatenated in name order, at 4M fixed seeded positions: 16 MB).
+    Some gradient reductions use atomics, so two runs agree only up to rounding that the steps amplify (B200, 1000 W, 3 warm-up +
+    10 timed steps, two pairs of runs: loss within 1.3e-3, parameters within 6e-3 relative L2)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    state = eng.trainable_state("param")
+    params = torch.cat([state[k].detach().float().reshape(-1) for k in sorted(state)])
+    if params.numel() > sample:
+        idx = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:sample].sort().values
+        params = params[idx.to(params.device)]
+    arrays = {"loss": loss.detach().float().reshape(1), "accuracy": acc.detach().float().reshape(1), "trainable_params": params}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_reference(args):
     rank, local_rank, world = dist_env()
     if rank != 0:
@@ -697,6 +716,8 @@ def run_ours(args):
     ms_per_step = ms / args.steps
     value = world * audio_s / (ms_per_step / 1e3)
     final_loss = loss.item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, acc, eng)              # before any later step overwrites the graph's loss buffer
     # ---------------- the same K steps again with a CUDA-event pair around every GEMM launch (roofline of the GEMM family);
     # kept out of the `value` region because ~900 extra event records per step cost ~3 % of host time
     for _ in range(2):                                               # the eager path's own allocator pool (the timed steps ran from graphs)
@@ -773,7 +794,7 @@ def run_ours(args):
             continue
     eager = None
     if world == 1 and not args.skip_eager and wl["batch"] is not None:
-        eager = eager_baseline(wl, enc, llm, lora, host_batch, dev, eng, audio_s, e2e_value, model=model)
+        eager = eager_baseline(wl, enc, llm, lora, host_batch, dev, eng, audio_s, e2e_value, steps=args.steps, warmup=max(args.warmup, 3), model=model)
     cb = None
     if world == 1 and not args.skip_cpu:
         cb, _ = cpu_reference(wl, steps=2, warmup=0, budget_s=25.0)
@@ -821,7 +842,11 @@ def main():
                                                               "-> gpurun_out/scale_breakdown_n{N}.json")
     ap.add_argument("--skip-recipe", action="store_true", help="skip the e2e_recipe leg (train() + DataLoader)")
     ap.add_argument("--skip-eager", action="store_true", help="skip the eager-HF-on-GPU baseline leg (B-EAGER)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (loss, accuracy, sampled trainable parameters)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

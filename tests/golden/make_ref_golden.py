@@ -1,9 +1,9 @@
 """Run the REFERENCE'S OWN hot path on the CPU and commit what it produced (tests/golden/ref_*.pt).
 
-    python tests/golden/make_ref_golden.py            # writes ref_tiny.pt, ref_collator.pt, ref_realwidth.pt
-    python tests/golden/make_ref_golden.py --check    # regenerates in memory and compares with the committed files
+    SLAM_LLM_REFERENCE=<checkout of the original SLAM-LLM> python tests/golden/make_ref_golden.py [--only NAME]   # writes ref_*.pt
+    SLAM_LLM_REFERENCE=<checkout of the original SLAM-LLM> python tests/golden/make_ref_golden.py --check        # compares instead
 
-Everything below `reference_step` executes /root/reference/src/slam_llm UNMODIFIED (imported through tests/ref_glue.py's
+Everything below `reference_step` executes the original project's src/slam_llm UNMODIFIED (imported through tests/ref_glue.py's
 stand-ins for the absent third-party packages):
     datasets/speech_dataset.py  SpeechDatasetJsonl.__getitem__ + collator (:86-291)  on fabricated WAV + jsonl files
     models/slam_model.py        setup_encoder (:68-116) -> models/encoder.py WhisperWrappedEncoder.load (:9-45)
@@ -11,7 +11,9 @@ stand-ins for the absent third-party packages):
                                 setup_encoder_projector (:223-236) -> models/projector.py
                                 slam_model.forward (:283-407) incl. utils/metric.py compute_accuracy
     optimizer                   torch.optim.AdamW(model.parameters(), lr, weight_decay) as pipeline/finetune.py:247-251
-The GPU box has no /root/reference: it only reads the committed fixtures (tests/test_ref_parity*.py).
+The tests only read the committed fixtures (tests/test_ref_pinning.py, tests/test_ref_parity_gpu.py).  To keep every file small, a
+tensor of more than FULL_MAX elements is stored as a probe (its norm and its first PROBE_HEAD elements), the parameters after the
+AdamW step as probes of AFTER_HEAD elements, and the projector output of the small cases at every AUDIO_TOKEN_STRIDE-th token.
 
 Weights come from the oracle's seeded initialisers (oracle/slam_oracle.py init_*) with the FROZEN matrices rounded to bf16
 (what the device stores, tests/parity_util.round_frozen), so a test can rebuild identical weights from the seeds alone.
@@ -34,10 +36,13 @@ sys.path.insert(0, ROOT)
 
 import ref_glue  # noqa: E402
 
-ref_glue.install()                                   # /root/reference/src first on sys.path, stand-ins installed
+ref_glue.install()                                   # the reference's src first on sys.path, stand-ins installed
 from omegaconf import OmegaConf  # noqa: E402  (the repo shim or the real package)
 from oracle import slam_oracle as so  # noqa: E402  (seeded initialisers + cfg dataclasses only; the arithmetic below is the reference's)
 from parity_util import round_frozen  # noqa: E402
+from ref_fixture import AUDIO_TOKEN_STRIDE  # noqa: E402
+
+FULL_MAX, PROBE_HEAD, AFTER_HEAD = 4096, 2048, 1024
 
 CASES = {
     # dh = 64, GQA 2:1, LoRA q/v, hidden 2048 (hard-coded in the reference projector, projector.py:11)
@@ -53,9 +58,9 @@ CASES = {
 # dynamic-frame recipe (datasets/speech_dataset_large.py): natural-length utterances (odd and even frame counts), right padding only,
 # batches formed by the window rule (:259-263) with a 260-token budget; the step runs on the first batch with >= 3 utterances
 CASES["tiny_dynamic"] = dict(CASES["tiny"], seed=4242)
-DYNAMIC = dict(max_frame_length=260,
+DYNAMIC = dict(max_frame_length=260, max_audio_length=3,
                utts=[(0.6131, "ASR", "ab"), (1.5075, "ST", "hello there"), (2.2506, "ASR", "c"), (0.9519, "ASR", "lorem ipsum"), (1.8107, "ST", "x y z"),
-                     (31.0, "ASR", "dropped: longer than max_audio_length"), (0.4006, "ASR", "q")],
+                     (3.1, "ASR", "dropped: longer than max_audio_length"), (0.4006, "ASR", "q")],
                prompts={"ASR": "Transcribe. ", "ST": "Translate the speech to German. "})
 
 UTTERANCES = {   # (seconds, target text, prompt) — two prompts so the collator left-pads (speech_dataset.py:224-236)
@@ -119,7 +124,8 @@ def dynamic_batches(case, tmp, mods, tokenizer):
         for task, prompt in DYNAMIC["prompts"].items():
             f.write(json.dumps({"task": task, "prompt": prompt}) + "\n")
     dc = OmegaConf.create(dict(train_scp_file_path=scp, dev_scp_file_path=scp, test_scp_file_path=scp, multitask_prompt_path=pp, append_info_tasks=[],
-                               prompt_style="USER: {}\n ASSISTANT:", mel_size=CASES[case]["enc"][0], input_type="mel", pad_or_trim=False, max_audio_length=30,
+                               prompt_style="USER: {}\n ASSISTANT:", mel_size=CASES[case]["enc"][0], input_type="mel", pad_or_trim=False,
+                               max_audio_length=DYNAMIC["max_audio_length"],
                                train_max_frame_length=DYNAMIC["max_frame_length"], eval_max_frame_length=DYNAMIC["max_frame_length"]))
     ds = mods["speech_dataset_large"].get_speech_dataset(dc, tokenizer, "train")
     groups = [list(items) for items in ds]
@@ -199,9 +205,9 @@ def reference_s2s_step() -> dict:
     import whisper
     from transformers import Qwen2Config, Qwen2ForCausalLM
     mods = ref_glue.reference_modules()
-    sys.path.insert(0, "/root/reference/examples/s2s")
+    sys.path.insert(0, os.path.join(ref_glue.REFERENCE, "examples", "s2s"))
     s2s_mod = importlib.import_module("model.slam_model_s2s")
-    assert s2s_mod.__file__.startswith("/root/reference/")
+    assert s2s_mod.__file__.startswith(os.path.abspath(ref_glue.REFERENCE))
     L, TV, AV = S2S["code_layer"], S2S["text_vocab"], S2S["audio_vocab"]
     enc, llm, proj = so.EncoderCfg(*S2S["enc"]), so.LlmCfg(*S2S["llm"]), so.ProjCfg(*S2S["proj"])
     assert llm.vocab == TV + L * AV
@@ -254,7 +260,7 @@ def reference_s2s_step() -> dict:
         if n == "llm.lm_head.weight":                                   # tied: the same tensor as the embedding (HF lists it once)
             continue
         g = p.grad.detach() if p.grad is not None else torch.zeros_like(p)
-        grads[n] = g.clone() if g.numel() <= 70000 else probe(g, 4096)
+        grads[n] = g.clone() if g.numel() <= FULL_MAX else probe(g, PROBE_HEAD)
     return dict(case="s2s", cfg=S2S, loss=outputs.loss.item(), text_acc=float(text_acc), layer_loss=[float(l) for l in layer_loss], grads=grads,
                 mel=probe(mel, 512), logits=probe(outputs.logits.detach(), 2048), trainable=sorted(grads))
 
@@ -276,8 +282,8 @@ def reference_step(case: str) -> dict:
             all_batches, pcm_all = dynamic_batches(case, tmp, mods, tokenizer)
             pick = next(i for i, b in enumerate(all_batches) if b["input_ids"].shape[0] >= 3)
             batch = all_batches[pick]
-            used, seen = [], 0                                       # utterances of the picked batch, in dataset order (the 31 s one is dropped)
-            kept = [i for i, (secs, _, _) in enumerate(DYNAMIC["utts"]) if secs <= 30]
+            used, seen = [], 0                                       # utterances of the picked batch, in dataset order (the too-long one is dropped)
+            kept = [i for i, (secs, _, _) in enumerate(DYNAMIC["utts"]) if secs <= DYNAMIC["max_audio_length"]]
             for bi, b in enumerate(all_batches):
                 n = b["input_ids"].shape[0]
                 if bi == pick:
@@ -321,11 +327,11 @@ def reference_step(case: str) -> dict:
     out["mel"] = probe(batch["audio_mel"], 512)
     if small:
         out["encoder_out"] = enc_out[:, :40].clone()                                   # first 40 frames of every utterance, all channels
-        out["audio_tokens"] = aud.clone()
+        out["audio_tokens"] = aud[:, ::AUDIO_TOKEN_STRIDE].clone()
         out["inputs_embeds"] = probe(embeds, 1024)
         out["label_logits"] = lab_logits.clone()
-        out["grads"] = {k: (v.clone() if v.numel() <= 70000 else probe(v, 4096)) for k, v in grads.items()}
-        out["after"] = {k: probe(v, 4096) for k, v in after.items()}
+        out["grads"] = {k: (v.clone() if v.numel() <= FULL_MAX else probe(v, PROBE_HEAD)) for k, v in grads.items()}
+        out["after"] = {k: probe(v, AFTER_HEAD) for k, v in after.items()}
     else:
         out["encoder_out"] = probe(enc_out)
         out["encoder_out_rows"] = enc_out[:, ::500, :64].clone()

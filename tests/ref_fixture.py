@@ -1,5 +1,5 @@
 """Helpers shared by the CPU pinning tests and the GPU parity tests that read the REFERENCE-RUN fixtures
-(tests/golden/ref_*.pt, produced by tests/golden/make_ref_golden.py from /root/reference's own code).  Test infrastructure."""
+(tests/golden/ref_*.pt, produced by tests/golden/make_ref_golden.py from the original project's own code).  Test infrastructure."""
 from __future__ import annotations
 
 import os
@@ -10,6 +10,7 @@ from oracle import slam_oracle as so
 from parity_util import round_frozen
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+AUDIO_TOKEN_STRIDE = 10          # the small fixtures keep every 10th projector output token (audio_tokens[:, ::10]) to stay small
 
 
 def load(name: str) -> dict:

@@ -1,8 +1,8 @@
-"""Run the REFERENCE'S OWN code for the hot path in this container (test infrastructure; never shipped, never on the GPU box).
+"""Run the REFERENCE'S OWN code for the hot path on the CPU (test infrastructure for tests/golden/make_ref_golden.py; never shipped).
 
-`/root/reference/src/slam_llm` imports third-party packages that are absent offline (peft, openai-whisper, soundfile,
-deepspeed, omegaconf).  This module installs small stand-ins for exactly the names the reference reaches for, puts
-`/root/reference/src` first on sys.path and imports the reference's modules UNMODIFIED:
+The original project's `src/slam_llm` (a checkout named by the SLAM_LLM_REFERENCE environment variable) imports third-party
+packages that are absent offline (peft, openai-whisper, soundfile, deepspeed, omegaconf).  This module installs small stand-ins
+for exactly the names the reference reaches for, puts its `src` first on sys.path and imports the reference's modules UNMODIFIED:
 
     slam_llm.models.slam_model      (setup_encoder / setup_llm / setup_encoder_projector / slam_model.forward, :68-407)
     slam_llm.models.encoder         (WhisperWrappedEncoder.load -> extract_variable_length_features, :13-45)
@@ -36,12 +36,13 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-REFERENCE_SRC = "/root/reference/src"
+REFERENCE = os.environ.get("SLAM_LLM_REFERENCE", "")                          # checkout of the original SLAM-LLM project
+REFERENCE_SRC = os.path.join(os.path.abspath(REFERENCE), "src") if REFERENCE else ""
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_SRC, "slam_llm"))
+    return bool(REFERENCE_SRC) and os.path.isdir(os.path.join(REFERENCE_SRC, "slam_llm"))
 
 
 # =====================================================================================================================
@@ -342,9 +343,10 @@ def _load_by_path(name: str, path: str) -> types.ModuleType:
 
 
 def install(extra_stubs: Iterable[str] = ()) -> None:
-    """Make `import slam_llm...` resolve to /root/reference/src with the stand-ins in place."""
+    """Make `import slam_llm...` resolve to the reference's src with the stand-ins in place."""
     if not reference_available():
-        raise RuntimeError("/root/reference is not present (GPU box): the reference-run fixtures are committed under tests/golden/")
+        raise RuntimeError("SLAM_LLM_REFERENCE does not name a checkout of the original SLAM-LLM project: the reference-run fixtures are "
+                           "committed under tests/golden/")
     loaded = sys.modules.get("slam_llm")
     if loaded is not None and not getattr(loaded, "__file__", "").startswith(REFERENCE_SRC):
         raise RuntimeError("the repo's slam_llm mirror is already imported in this process; use a dedicated process")

@@ -20,7 +20,6 @@ from omegaconf import DictConfig, ListConfig, OmegaConf  # noqa: E402
 
 # ------------------------------------------------------------------------------------------------- config surface
 def test_omegaconf_merge_and_access_like_the_recipes():
-    sys.path.insert(0, "/root/reference/examples/asr_librispeech") if os.path.isdir("/root/reference") else None
     from dataclasses import dataclass, field
     from typing import List, Optional
 
@@ -378,50 +377,6 @@ def test_bench_gemm_traffic_parser_and_fallback(tmp_path, monkeypatch):
     monkeypatch.setattr("shutil.which", lambda name: None)
     monkeypatch.setattr(os.path, "exists", lambda p, _orig=os.path.exists: False if str(p).endswith("/ncu") else _orig(p))
     assert bench.measure_gemm_traffic("c3") == (None, "ncu not found")
-
-
-# ------------------------------------------------------------------------------------------------- reference recipe files, unchanged
-@pytest.mark.skipif(not os.path.isdir("/root/reference/examples/asr_librispeech"), reason="reference tree not present (GPU box)")
-def test_reference_recipe_files_import_unchanged_against_the_mirror(monkeypatch):
-    """examples/asr_librispeech/{finetune_asr.py, asr_config.py, model/slam_model_asr.py} import slam_llm by name; they must
-    load against src/slam_llm without modification (hydra / omegaconf via the offline shims)."""
-    rec = "/root/reference/examples/asr_librispeech"
-    monkeypatch.syspath_prepend(rec)
-    from slam_llm.utils.dataset_utils import load_module_from_py_file
-    asr_config = load_module_from_py_file(os.path.join(rec, "asr_config.py"))
-    sys.modules["asr_config"] = asr_config
-    ft = load_module_from_py_file(os.path.join(rec, "finetune_asr.py"))
-    cfg = OmegaConf.merge(ft.RunConfig(), OmegaConf.from_dotlist(["++train_config.use_peft=true", "++model_config.encoder_name=whisper"]))
-    assert cfg.train_config.peft_config.r == 8 and cfg.model_config.encoder_projector == "linear" and cfg.dataset_config.mel_size == 80
-    assert cfg.dataset_config.file == "src/slam_llm/datasets/speech_dataset.py:get_speech_dataset"
-    assert os.path.isfile(os.path.join(ROOT, cfg.dataset_config.file.split(":")[0]))      # default path resolves from the repo root
-    model_mod = load_module_from_py_file(os.path.join(rec, "model", "slam_model_asr.py"))
-    import slam_llm.models.slam_model as sm
-    assert issubclass(model_mod.slam_model_asr, sm.slam_model) and callable(model_mod.model_factory)
-    from slam_llm.pipeline.finetune import main
-    assert ft.train is main
-
-
-def test_reference_model_factory_reaches_the_b200_engine(tmp_path, monkeypatch):
-    """The reference's OWN examples/asr_librispeech/model/slam_model_asr.py:model_factory, loaded through the plugin loader exactly like
-    finetune.main does (utils/model_utils.py:4-29), runs against the mirror: tokenizer from llm_path, then setup_encoder hands over to the
-    B200 engine — which on this CPU-only box refuses loudly (no CPU fallback).  On a GPU box the same call chain is exercised by
-    tests/test_recipe_gpu.py through a plugin of the same shape (the reference file itself cannot travel to the GPU box)."""
-    import logging
-    import torch
-    from recipe_util import make_llm_dir, run_config
-    from slam_llm.utils.model_utils import get_custom_model_factory
-    if torch.cuda.is_available():
-        pytest.skip("CPU-box check of the refusal path")
-    rec = "/root/reference/examples/asr_librispeech/model/slam_model_asr.py"
-    if not os.path.isfile(rec):
-        pytest.skip("/root/reference is only present in the build container")
-    llm_dir = make_llm_dir(str(tmp_path / "llm"))
-    cfg = run_config(llm_dir, "unused.jsonl", str(tmp_path), rec + ":model_factory", "src/slam_llm/datasets/speech_dataset.py:get_speech_dataset")
-    factory = get_custom_model_factory(cfg.model_config, logging.getLogger())
-    assert factory.__module__ != "recipe_model" and factory.__code__.co_filename == rec
-    with pytest.raises(RuntimeError, match="CUDA"):
-        factory(cfg.train_config, cfg.model_config, metric="acc")
 
 
 # ------------------------------------------------------------------------------------------------- dynamic-frame batching (config 3)

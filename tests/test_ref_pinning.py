@@ -1,14 +1,13 @@
 """Pin the oracle (and the host-side collator mirror) to outputs of the REFERENCE'S OWN code.
 
-tests/golden/ref_*.pt were produced by tests/golden/make_ref_golden.py, which imports /root/reference/src/slam_llm unmodified
+tests/golden/ref_*.pt were produced by tests/golden/make_ref_golden.py, which imports the original project's src/slam_llm unmodified
 (datasets/speech_dataset.py __getitem__ + collator, models/slam_model.py setup_* + slam_model.forward, models/encoder.py,
 models/projector.py, utils/metric.py, utils/config_utils.generate_peft_config) over HF LlamaForCausalLM and stand-ins for the
 absent peft / openai-whisper packages (tests/ref_glue.py), runs one training step on the CPU and stores what came out.
 These tests rebuild the same weights from the seeds, feed the oracle the same collated batch and require fp32-level agreement:
     loss rel <= 1e-5, activations / logits rel-max <= 1e-4, gradients rel-L2 <= 1e-4.
-A further test re-runs the generator with --check when /root/reference is present (this container; not the GPU box)."""
+`make_ref_golden.py --check` re-runs the original code and compares it with the committed fixtures."""
 import os
-import subprocess
 import sys
 
 import pytest
@@ -39,7 +38,7 @@ def _oracle_vs_fixture(fix, small: bool):
     lab = ref["logits"][:, :-1][rows]
     if small:
         assert rf.rel_max(ref["encoder_out"][:, :40], fix["encoder_out"]) < FP32["act"]
-        assert rf.rel_max(ref["audio_tokens"], fix["audio_tokens"]) < FP32["act"]
+        assert rf.rel_max(ref["audio_tokens"][:, ::rf.AUDIO_TOKEN_STRIDE], fix["audio_tokens"]) < FP32["act"]
         assert rf.rel_max(lab, fix["label_logits"]) < FP32["act"]
         rf.check_probe(ref["inputs_embeds"], fix["inputs_embeds"], norm_rel=1e-5, head_rel=1e-4, what="inputs_embeds")
     else:
@@ -190,7 +189,8 @@ def test_dynamic_dataset_mirror_reproduces_the_reference_batches(tmp_path):
     pp.write_text("".join(json.dumps({"task": t, "prompt": p}) + "\n" for t, p in dyn["prompts"].items()))
     dc = OmegaConf.create(dict(train_scp_file_path=str(scp), dev_scp_file_path=str(scp), test_scp_file_path=str(scp), multitask_prompt_path=str(pp),
                                append_info_tasks=[], prompt_style="USER: {}\n ASSISTANT:", mel_size=80, input_type="mel", pad_or_trim=False,
-                               max_audio_length=30, train_max_frame_length=dyn["max_frame_length"], eval_max_frame_length=dyn["max_frame_length"]))
+                               max_audio_length=dyn["max_audio_length"], train_max_frame_length=dyn["max_frame_length"],
+                               eval_max_frame_length=dyn["max_frame_length"]))
     ds = get_speech_dataset(dc, CharTokenizer(512), "train")
     got = [ds.collator(items) for items in ds]
     assert len(got) == len(fix["all_batches"])
@@ -239,13 +239,3 @@ def test_audio_dataset_mirror_matches_the_reference_audio_dataset(tmp_path):
         else:
             assert torch.equal(batch[k].to(v.dtype), v), k
 
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src/slam_llm"), reason="/root/reference is only present in the build container")
-def test_fixtures_regenerate_from_the_reference_code():
-    """Re-run the reference's own code (dedicated process: its `slam_llm` package shadows this repo's mirror) and compare with the
-    committed fixtures.  The real-width case is left to `make_ref_golden.py --check --only realwidth` (3 min)."""
-    for only in ("tiny", "collator", "s2s", "audio_dataset"):   # "tiny" matches ref_tiny, ref_tiny_cov1d_all and ref_tiny_dynamic
-        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "make_ref_golden.py"), "--check", "--only", only],
-                           capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
-        assert "ok ref_" in r.stdout
