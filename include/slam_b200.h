@@ -135,7 +135,10 @@ int slam_layernorm(const void* x_bf16, const float* w, const float* b, void* y_b
  *   lse f32 [B,Hq,Sq] (log-sum-exp, natural log) or NULL.  out bf16 [B,Sq,Hq,dh] with row stride ldo.
  * Replaces whisper MultiHeadAttention.qkv_attention and HF LlamaAttention (eager softmax).
  * Kernels: tcgen05 / TMEM flash attention for dh = 64 / 128 with Sq == Sk >= 64 (forward) and dh = 128 (backward);
- * mma.sync flash kernels for every other shape - same arguments, same results within bf16 rounding. */
+ * mma.sync flash kernels for every other shape - same arguments, same results within bf16 rounding.
+ * Masking contract (both kernel families): a query row that sees no key (every key masked, or left padding under the causal mask)
+ * gets out = 0 and lse = 0 exactly, and dQ = 0 exactly in the backward; a masked key gets dK = dV = 0 exactly, and the values
+ * stored at masked K / V positions never reach out or lse (any finite values give bit-identical results). */
 typedef struct slam_attn_args {
   const void* q; int64_t ldq;   /* row stride between consecutive tokens, elements */
   const void* k; int64_t ldk;

@@ -301,6 +301,10 @@ def _ref_attn(q, k, v, causal, scale, key_mask):
     (1, 700, 8, 8, 128, True, False),      # several key tiles, causal tile skipping
     (2, 200, 4, 4, 64, False, True),       # key mask without causal
     (1, 40, 4, 2, 64, True, True),         # short: mma.sync kernel
+    # tile and dispatch edges (tcgen05 from S = 64, 128-key / 128-query tiles; mma.sync below): with B = 3 the 128-row TMA tiles of
+    # samples 0 and 1 reach into the next sample's rows
+    *[(3, S, 8, 2, 128, True, True) for S in (63, 64, 127, 128, 129, 255, 257)],
+    *[(3, S, 4, 4, 64, False, False) for S in (63, 64, 127, 128, 129, 255, 257)],
 ])
 def test_attention_fwd_bwd(ops, B, S, Hq, Hkv, dh, causal, masked):
     qkv = rnd(B * S, (Hq + 2 * Hkv) * dh, seed=27)  # fused QKV buffer, used in place
@@ -605,3 +609,74 @@ def test_utilities(ops):
     dstt = torch.zeros(3, 40, 64, device=dev(), dtype=BF16)
     ops.pack2d(src, dstt, batch=3, rows=16, cols=40, src_bs=16 * 40, src_ld=40, dst_bs=40 * 64, dst_ld=64, dst_off=32, transpose=True)
     assert torch.equal(dstt[:, :, 32:48], src.transpose(1, 2).to(BF16))
+
+
+# ----------------------------------------------------------------------------------------------- full fine-tune reductions (fp64 references)
+# The kernels below sum fp32 terms in a fixed tree: a run of terms per thread, 8 row lanes, then one fp32 atomic per row slice (at most 64).
+# Whatever the order, the rounding error of an n-term fp32 sum is at most about n * 2^-24 * sum|terms| (recursive summation bound); every
+# path here has n < 170, so |err| <= 1e-5 * sum|terms| holds with margin.
+SUM_BOUND = 1e-5
+
+
+@pytest.mark.parametrize("rows", [1, 257, 1604, 16400])
+@pytest.mark.parametrize("d", [896, 900, 4096])
+def test_rmsnorm_wgrad(ops, rows, d):
+    """dw[c] += sum_r dy[r,c] * x[r,c] * rstd[r], accumulated into a non-zero dw; 16400 rows use the 64-way row split."""
+    dy, x = rnd(rows, d, seed=110), rnd(rows, d, scale=2.0, seed=111)
+    g = torch.Generator(device="cuda").manual_seed(112)
+    rstd = torch.rand(rows, device=dev(), generator=g) * 1.5 + 0.5
+    dw0 = rnd(d, dtype=F32, seed=113)
+    dw = ops.rmsnorm_wgrad(dy, x, rstd, dw0.clone())
+    terms = dy.double() * x.double() * rstd.double()[:, None]
+    ref = dw0.double() + terms.sum(0)
+    bound = SUM_BOUND * (dw0.double().abs() + terms.abs().sum(0))
+    assert ((dw.double() - ref).abs() <= bound).all(), ((dw.double() - ref).abs() / bound).max().item()
+
+
+def test_embed_grad(ops):
+    """dE[max(id, 0)] += dx[r] for text rows (modality mask 0): repeated ids accumulate, -1 goes to row 0, ids >= vocab and audio rows are
+    skipped.  Rows nobody writes keep their value bit for bit; the guard rows after the table are never written."""
+    V, d, rows = 1000, 896, 300
+    g = torch.Generator(device="cuda").manual_seed(120)
+    ids = torch.randint(0, 40, (rows,), device=dev(), generator=g)        # 40 distinct ids over 300 rows: many repeats
+    ids[::7] = -1
+    ids[5::11] = V + 3
+    ids[6] = V
+    mask = torch.zeros(rows, dtype=torch.uint8, device=dev())
+    mask[100:160] = 1
+    dx = rnd(rows, d, seed=121)
+    table = torch.full((V + 8, d), float("nan"), device=dev(), dtype=F32)
+    table[:V] = rnd(V, d, dtype=F32, seed=122)
+    de0 = table[:V].clone()
+    ops.embed_grad(ids, mask, dx, table[:V])
+    keep = (mask == 0) & (ids < V)
+    tgt = ids.clamp_min(0)[keep]
+    ref, absum = de0.double(), de0.double().abs()
+    ref.index_add_(0, tgt, dx.double()[keep])
+    absum.index_add_(0, tgt, dx.double().abs()[keep])
+    assert ((table[:V].double() - ref).abs() <= SUM_BOUND * absum).all()
+    untouched = torch.ones(V, dtype=torch.bool, device=dev())
+    untouched[tgt] = False
+    assert torch.equal(table[:V][untouched], de0[untouched])
+    assert torch.isnan(table[V:]).all()
+
+
+@pytest.mark.parametrize("batch,rows,cols", [(3, 45, 77), (2, 100, 33), (1, 31, 1), (4, 64, 96)])
+def test_transpose_f32_batched(ops, batch, rows, cols):
+    """dst[b][j][i] = src[b][i][j], sides not multiples of the 32 x 32 tile: pure data movement, exact; every element written."""
+    src = rnd(batch, rows, cols, dtype=F32, seed=130)
+    dst = torch.full((batch, cols, rows), float("nan"), device=dev(), dtype=F32)
+    ops.transpose_f32_batched(src, dst, batch, rows, cols)
+    assert torch.equal(dst, src.transpose(1, 2))
+
+
+@pytest.mark.parametrize("rows,cols", [(6007, 200), (20000, 1000), (1, 72)])
+def test_colsum(ops, rows, cols):
+    """out[c] = sum_r x[r,c] on a column slice of a wider buffer (row stride != cols) into a NaN-filled out: the kernel zeroes it first;
+    20000 rows use the 64-way row split."""
+    big = rnd(rows, cols + 24, scale=3.0, seed=140)
+    x = big[:, 8:8 + cols]
+    out = torch.full((cols,), float("nan"), device=dev(), dtype=F32)
+    ops.colsum(x, out)
+    ref = x.double().sum(0)
+    assert ((out.double() - ref).abs() <= SUM_BOUND * x.double().abs().sum(0)).all()
